@@ -31,6 +31,7 @@ for p in (ROOT, os.path.join(ROOT, "metavoice-src_b200")):
     if p not in sys.path:
         sys.path.insert(0, p)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 T_PROMPT, N_NEW = 48, 750
@@ -159,6 +160,18 @@ def tokens_generated(model, utts):
     return out
 
 
+def generated_tokens(model, utts, n_new):
+    """The token ids the last decode left in every utterance slot, as mvb_s1_fetch hands them to a caller: int32 [utts, n_new]."""
+    import ctypes as C
+    from mvb200 import _lib
+    out = np.zeros((utts, n_new), np.int32)
+    for u in range(utts):
+        n, d = C.c_int32(0), C.c_int32(0)
+        _lib.check(model._lib.mvb_s1_fetch(model.handle, u, out[u].ctypes.data_as(C.c_void_p), n_new, C.byref(n), C.byref(d),
+                                           model._stream()))
+    return out
+
+
 def step_roofline(model, lens, n_new, reps, device):
     """One persistent launch of `reps` decode positions around the middle of the utterance (CUDA events on the launching
     stream): algorithmic bytes = reps x weights + K/V of every cached position read + the appended position written."""
@@ -207,7 +220,11 @@ def main():
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--skip-pipeline", action="store_true")
     ap.add_argument("--skip-configs", action="store_true", help="skip the batch-8 / long-form legs (BASELINE configs[2], [3])")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the token ids of the last timed step to DIR/stage1_tokens.npy "
+                                                          "(float32 [utts-per-gpu, 750]; one file per rank when --gpus > 1)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
 
@@ -273,6 +290,10 @@ def main():
     launches = model._lib.mvb_s1_launch_count(model.handle) - lc0
     ms = e0.elapsed_time(e1)
     assert tokens_generated(model, utts) == [N_NEW] * utts
+    if a.dump_outputs:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        name = "stage1_tokens" if world == 1 else f"stage1_tokens_rank{rank}"
+        np.save(os.path.join(a.dump_outputs, name + ".npy"), generated_tokens(model, utts, N_NEW).astype(np.float32))
 
     # ---- decode roofline: one persistent launch of `reps` positions at mid-utterance context ----
     reps = 200

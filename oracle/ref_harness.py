@@ -35,11 +35,6 @@ def _resolve_root() -> str:
 REFERENCE_ROOT = _resolve_root()
 
 
-def available() -> bool:
-    """The reference tree itself is mounted (build container): gates the live-reference tests."""
-    return os.path.isdir("/root/reference/fam/llm") or bool(os.environ.get("MVB_REFERENCE_ROOT"))
-
-
 def runnable() -> bool:
     """The reference's code can be imported here (mounted tree or the vendored copy): gates bench.py's reference arm."""
     return os.path.isdir(os.path.join(REFERENCE_ROOT, "fam", "llm"))

@@ -12,9 +12,8 @@ legs may import this file.  It follows, function by function:
   * ``fam/llm/fast_inference_utils.py:123-228``  prefill / decode_one_token / decode_n_tokens / generate
   * ``fam/llm/fast_inference_utils.py:246-278``  checkpoint key mapping
 
-Pinning: ``tests/test_oracle_pinned.py`` checks this port against the reference's own code imported
-from /root/reference (when that tree is present) and against the committed golden vectors produced
-by ``oracle/make_golden.py`` from the reference's own code (always).
+Pinning: ``tests/test_oracle_pinned.py`` checks this port against the committed golden vectors produced
+by ``oracle/make_golden.py`` and ``oracle/make_golden_reference.py`` from the reference's own code.
 """
 from __future__ import annotations
 

@@ -8,8 +8,8 @@
   * ``FlattenedInterleavedEncodec2Codebook.decode``          fam/llm/adapters/flattened_encodec.py:8-32
   * ``TiltedEncodec.decode``                                 fam/llm/adapters/tilted_encodec.py:8-39
 
-Pinned by tests/test_oracle_pinned_stage2.py against the reference's own ``GPT`` (live when /root/reference is
-mounted) and against tests/golden/stage2.npz produced from it by oracle/make_golden_stage2.py.
+Pinned by tests/test_oracle_pinned_stage2.py against tests/golden/stage2.npz, produced from the reference's own
+``GPT`` by oracle/make_golden_stage2.py.
 """
 from __future__ import annotations
 

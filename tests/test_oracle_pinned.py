@@ -1,12 +1,12 @@
-"""CPU: the oracle restatement (oracle/stage1_port.py) against (a) the committed golden vectors that were
-produced by the reference's own code (oracle/make_golden.py) and (b) the reference itself when the tree is
-mounted.  If these fail, no GPU parity claim means anything."""
+"""CPU: the oracle restatement (oracle/stage1_port.py) against the committed golden vectors that were produced by
+the reference's own code (oracle/make_golden.py, oracle/make_golden_reference.py).  If these fail, no GPU parity
+claim means anything."""
 import numpy as np
 import pytest
 import torch
 
 from mvb200 import synth
-from oracle import ref_harness, stage1_port as P
+from oracle import stage1_port as P
 
 
 def _load(golden_dir, name):
@@ -92,22 +92,20 @@ def test_prompt_too_long_raises():
         P.generate(m, synth.synthetic_prompt(2048), synth.synthetic_speaker(), guidance_scale=3.0, temperature=1.0)
 
 
-@pytest.mark.skipif(not ref_harness.available(), reason="reference tree not mounted (GPU box)")
-def test_port_matches_live_reference():
+def test_port_matches_live_reference(golden_dir):
+    """The reference's own Transformer forward and generate() on the same weights and inputs, as recorded by
+    oracle/make_golden_reference.py."""
+    g = _load(golden_dir, "reference_checks")
     d = synth.TINY
     sd = synth.stage1_state_dict(d, 3)
-    ref = ref_harness.build_reference_model(sd, d, torch.float32)
+    assert synth.state_dict_checksum(sd) == pytest.approx(float(g["s1_checksum"]), rel=0, abs=1e-9)
     m = P.Stage1Oracle(sd, d.n_head, d.norm_eps, torch.float32); m.setup_caches()
-    prompt = synth.synthetic_prompt(9, seed=5); spk = synth.synthetic_speaker(seed=2)
+    prompt = torch.from_numpy(g["s1_prompt"]); spk = torch.from_numpy(g["s1_spk"])
     idx = prompt.view(1, -1).repeat(2, 1)
     with torch.no_grad():
-        a = ref(idx, spk, torch.arange(9)); b = m.forward(idx, spk, torch.arange(9))
+        a = torch.from_numpy(g["s1_logits"]); b = m.forward(idx, spk, torch.arange(9))
     assert (a - b).abs().max() < 1e-5
-    fiu = ref_harness.reference_functions()
-    ref2 = ref_harness.build_reference_model(sd, d, torch.float32)
-    kw = dict(temperature=torch.tensor(0.8), top_p=torch.tensor(0.9), guidance_scale=torch.tensor(2.0), top_k=None)
-    torch.manual_seed(5)
-    ya = fiu.generate(ref2, prompt, spk, max_new_tokens=12, end_of_audio_token=9999, **kw)
+    ya = torch.from_numpy(g["s1_tokens"])
     m2 = P.Stage1Oracle(sd, d.n_head, d.norm_eps, torch.float32); m2.setup_caches()
     torch.manual_seed(5)
     yb = P.generate(m2, prompt, spk, max_new_tokens=12, end_of_audio_token=9999, temperature=0.8, top_p=0.9,

@@ -1,11 +1,11 @@
-"""CPU: stage-2 oracle restatement vs golden vectors from the reference's own GPT (and vs the live reference)."""
+"""CPU: stage-2 oracle restatement vs golden vectors from the reference's own GPT, adapters and input builder."""
 import numpy as np
 import pytest
 import torch
 
 from mvb200 import synth
 from mvb200.second_stage import build_stage2_input, flattened_interleaved_decode, tilted_decode
-from oracle import ref_harness, stage2_port as P
+from oracle import stage2_port as P
 
 
 @pytest.mark.parametrize("tag,dims", [("tiny", synth.S2_TINY), ("full", synth.S2_FULL)])
@@ -38,16 +38,15 @@ def test_adapters_match_oracle_and_reference_semantics():
         assert codes[0] == [3, 4, 5] and codes[2] == [9, 9, 2]   # "first-N-valid" truncation (tilted_encodec.py:31-37)
 
 
-@pytest.mark.skipif(not ref_harness.available(), reason="reference tree not mounted (GPU box)")
-def test_adapters_match_live_reference():
-    ref_harness._import_reference()
-    from fam.llm.adapters import FlattenedInterleavedEncodec2Codebook, TiltedEncodec
-    g = torch.Generator().manual_seed(0)
-    flat = torch.randint(0, 2562, (300,), generator=g).tolist()
-    a = FlattenedInterleavedEncodec2Codebook(end_of_audio_token=1024).decode([flat])
+def test_adapters_match_live_reference(golden_dir):
+    """What the reference's own FlattenedInterleavedEncodec2Codebook.decode and TiltedEncodec.decode return, as recorded
+    by oracle/make_golden_reference.py."""
+    g = np.load(f"{golden_dir}/reference_checks.npz")
+    flat = g["flat_in"].tolist()
+    a = (g["flat_text"].tolist(), [g["flat_cb0"].tolist(), g["flat_cb1"].tolist()])
     assert tuple(a) == tuple(flattened_interleaved_decode(flat))
-    hier = torch.randint(0, 1100, (8, 200), generator=g).tolist()
-    b = TiltedEncodec(end_of_audio_token=1024).decode(hier)
+    hier = g["hier_in"].tolist()
+    b = (g["hier_text"].tolist(), g["hier_codes"].tolist())
     assert tuple(b) == tuple(tilted_decode(hier))
 
 
@@ -73,19 +72,12 @@ def test_product_input_builder_matches_reference_golden(golden_dir, tag):
         assert np.array_equal(P.build_input(g[f"{tag}_text_{i}"].tolist(), *g[f"{tag}_codes_{i}"].tolist(), bs).numpy(), ref[i])
 
 
-@pytest.mark.skipif(not ref_harness.available(), reason="reference tree not mounted (GPU box)")
-def test_product_input_builder_matches_live_reference():
-    import importlib.util
-    import os
-    spec = importlib.util.spec_from_file_location("mk_s2in", os.path.join(os.path.dirname(P.__file__), "make_golden_stage2_input.py"))
-    mk = importlib.util.module_from_spec(spec); spec.loader.exec_module(mk)
+def test_product_input_builder_matches_live_reference(golden_dir):
+    """The tensor the reference's own Model.non_causal_sample builds for three texts, as recorded by
+    oracle/make_golden_reference.py."""
     from mvb200.tokenise import TrainedBPETokeniser
     tok = TrainedBPETokeniser(**synth.synthetic_tokenizer_meta(n_text_tokens=512, offset=1025))
-    Model = mk.reference_model_class()
-    g = torch.Generator().manual_seed(77)
-    texts = ["a b c", "the quick brown fox", "x"]
-    codes = [torch.randint(0, 1024, (1, 2, n), generator=g) for n in (10, 300, 255)]
-    in_x = mk.reference_in_x(Model, tok, texts, codes, 256)
-    for i in range(3):
-        got = build_stage2_input(tok.encode(texts[i]), codes[i][0].tolist(), 256)
-        assert torch.equal(got.long(), in_x[i])
+    g = np.load(f"{golden_dir}/reference_checks.npz")
+    for i, text in enumerate(g["s2_texts"].tolist()):
+        got = build_stage2_input(tok.encode(text), g[f"s2_codes_{i}"].tolist(), 256)
+        assert torch.equal(got.long(), torch.from_numpy(g[f"s2_in_x_{i}"]))

@@ -5,7 +5,7 @@ import pytest
 import torch
 
 from mvb200 import synth
-from oracle import ref_harness, speaker_port as P
+from oracle import speaker_port as P
 
 
 def test_oracle_network_and_slicing_match_reference_golden(golden_dir):
@@ -24,16 +24,16 @@ def test_oracle_network_and_slicing_match_reference_golden(golden_dir):
     assert np.array_equal(slaney_mel_filterbank(16000, 400, 40), P.mel_filterbank())
 
 
-@pytest.mark.skipif(not ref_harness.available(), reason="reference tree not mounted (GPU box)")
-def test_partial_slices_match_live_reference():
-    ref_harness._import_reference()
-    from fam.quantiser.audio.speaker_encoder.model import SpeakerEncoder as Ref
+def test_partial_slices_match_live_reference(golden_dir):
+    """The slices the reference's own SpeakerEncoder.compute_partial_slices returns, as recorded by
+    oracle/make_golden_reference.py."""
     from mvb200.speaker_encoder import SpeakerEncoder
+    g = np.load(f"{golden_dir}/reference_checks.npz")
     for n in (16000, 25601, 102400, 480000, 777777):
         for rate, cov in ((1.3, 0.75), (2.0, 0.5)):
-            a, b = Ref.compute_partial_slices(n, rate, cov), SpeakerEncoder.compute_partial_slices(n, rate, cov)
-            assert [(s.start, s.stop) for s in a[0]] == [(s.start, s.stop) for s in b[0]]
-            assert [(s.start, s.stop) for s in a[1]] == [(s.start, s.stop) for s in b[1]]
+            a, b = (g[f"spk_{n}_{rate}_{cov}_wav"], g[f"spk_{n}_{rate}_{cov}_mel"]), SpeakerEncoder.compute_partial_slices(n, rate, cov)
+            assert [tuple(s) for s in a[0].tolist()] == [(s.start, s.stop) for s in b[0]]
+            assert [tuple(s) for s in a[1].tolist()] == [(s.start, s.stop) for s in b[1]]
 
 
 def test_wav_reader_resampler_trimmer(tmp_path):
